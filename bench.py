@@ -2,7 +2,7 @@
 """Benchmark of the NES generation hot path (BASELINE.json: generations/s and policy-evals/s, pop 64k).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--pop 65536] [--hidden 256] [--tape-len 256] [--precision fp32|f16|f16x3]
+                    [--pop 65536] [--hidden 256] [--tape-len 256] [--precision fp32|f16|f16x3] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (one rank per GPU, NCCL)
 
 A "step" is one NES generation (natural_es.py:62-96) over synthetic inputs: sample eps for the whole
@@ -37,6 +37,9 @@ import time
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
+# the tree may be read-only where the benchmark runs: no bytecode caches beside the sources, here or in the CPU legs
+sys.dont_write_bytecode = True
+os.environ['PYTHONDONTWRITEBYTECODE'] = '1'
 
 import numpy as np  # noqa: E402
 
@@ -61,6 +64,10 @@ def parse():
     ap.add_argument('--cpu-sample', type=int, default=0, help='members per CPU-baseline step (0 = auto)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed generation of the headline workload computed (fitness, theta, update, '
+                         'gradient partial sum) as DIR/<name>.npy, float32; inputs are seeded, so runs with the same '
+                         'arguments compare output for output')
     return ap.parse_args()
 
 
@@ -233,6 +240,19 @@ class ClockSampler:
                 'samples': len(sm)}
 
 
+DUMP_MAX_ELEMS = 3 << 20      # per array: 12 MiB of float32, so the four dumped arrays stay under 64 MB
+
+
+def dump_outputs(outdir, arrays):
+    """Write each device array as outdir/<name>.npy; one larger than DUMP_MAX_ELEMS is cut to a fixed, seeded sample."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, t in arrays.items():
+        x = t.detach().cpu().numpy().astype(np.float32).reshape(-1)
+        if x.size > DUMP_MAX_ELEMS:
+            x = x[np.sort(np.random.RandomState(0).choice(x.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(outdir, name + '.npy'), x)
+
+
 def build_hash():
     """Identity of the library the numbers were taken on (keys profiles/roofline_traffic.json)."""
     import hashlib
@@ -309,14 +329,18 @@ def run_ours(a):
                         device=dev, use_graph=not a.no_graph)
         return eng, env, theta0
 
-    def measure_nes(d0, H, A, T, N, precision, steps, warmup):
-        """Device-resident generations of one configuration + its dominant kernel alone -> (dict, engine, env)."""
+    def measure_nes(d0, H, A, T, N, precision, steps, warmup, outputs=None):
+        """Device-resident generations of one configuration + its dominant kernel alone -> (dict, engine, env).
+        `outputs`, if given, receives copies of what the last timed generation left for its caller."""
         eng, env, _ = make_engine(d0, H, A, T, N, precision)
         P = eng.P
         for _ in range(max(warmup, 3)):
             eng.generation()
         total_ms, _ = timed(eng.generation, steps)
         ms_per_step = max_over_ranks(total_ms) / steps
+        if outputs is not None:
+            outputs.update(fitness=eng.fitness_all.clone(), theta=eng.theta.clone(), update=eng.update.clone(),
+                           partial=eng.partial.clone())
 
         def eval_only():
             eng.k.nes_eval(eng.theta, eng.obs, eng.target, hidden=H, sigma=eng.sigma, clip=eng.clip, seed=eng.seed,
@@ -379,8 +403,11 @@ def run_ours(a):
     # ================================ headline workload ================================
     d0, H, A, T, N = a.state_dim, a.hidden, a.action_dim, a.tape_len, a.pop
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    main, eng, env = measure_nes(d0, H, A, T, N, a.precision, a.steps, a.warmup)
+    outputs = {} if a.dump_outputs else None
+    main, eng, env = measure_nes(d0, H, A, T, N, a.precision, a.steps, a.warmup, outputs)
     clocks = sampler.stop() if sampler else None
+    if outputs and rank == 0:
+        dump_outputs(a.dump_outputs, outputs)
     P = eng.P
     ms_per_step, value, roofline = main['ms_per_step'], main['value'], main['roofline']
 
