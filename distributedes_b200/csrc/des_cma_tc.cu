@@ -1,17 +1,23 @@
 // CMA-ES rank-mu covariance term on the tensor cores:  dC = sum_k w_k y_k y_k^T = Y^T diag(w) Y   (the arithmetic inside
 // es.tell, cma_es.py:90; Hansen tutorial arXiv:1604.00772 eq. 47) as a symmetric rank-k update with split-fp16 operands.
 //
-//   Z  = diag(sqrt|w|) Y           (so that dC = Zs^T Z with Zs = diag(sign w) Z; both operands are O(|y|): no scaling)
+//   Z  = diag(sqrt|w|) Y S         (so that dC = S^-1 (Zs^T Z) S^-1 with Zs = diag(sign w) Z)
+//   S  = diag(2^e_j)               per-coordinate power of two: max_k |Z_kj| lands in [2^14, 2^15).  Coordinate j of y has
+//                                  scale sqrt(C_jj), which CMA-ES learns and which spreads over many decades on ill-conditioned
+//                                  problems; unscaled, small coordinates lose lo to fp16 subnormals and large ones overflow hi
+//   exponents  Y [lambda][n] fp32 -> e [n] int32 (one coalesced read of Y)
 //   pre-pass   Y [lambda][n] fp32 -> Zs_hi, Zs_lo, Z_hi, Z_lo  [n][lambda_pad] fp16, k contiguous (K-major), x = hi + lo
 //   main       per 128 x 256 output tile touching the upper triangle:  D += A_hi B_hi^T + A_lo B_hi^T + A_hi B_lo^T
 //              (tcgen05.mma kind::f16, fp32 accumulation in TMEM; the dropped lo*lo term is 2^-22 relative), operand
 //              tiles brought in by TMA (cp.async.bulk.tensor.2d, SWIZZLE_128B) through a two-stage mbarrier pipeline:
-//              warp 0 = TMA producer, warp 1 = MMA issuer (+ TMEM allocation), warps 2-5 = epilogue (tcgen05.ld -> global)
+//              warp 0 = TMA producer, warp 1 = MMA issuer (+ TMEM allocation), warps 2-5 = epilogue (tcgen05.ld, times
+//              2^-e_i then 2^-e_j: both exact, -> global)
 //   output     the full symmetric matrix (upper entry written to both sides: exactly symmetric), or the packed
 //              upper-triangular tiles of des_cma_rank_mu_packed (the payload of the cross-rank sum)
 //
 // The fp32 FFMA kernel of des_cma.cu (36 % of the CUDA-core peak in round 1) stays as the small-n / no-workspace path.
-// Accuracy: measured against the fp64 restatement in tests/test_gpu_cma.py at the same 1e-5 (both norms) bar.
+// Accuracy: measured against the fp64 restatement in tests/test_gpu_cma.py at the same 1e-5 (both norms) bar, and entry by
+// entry (|err_ij| <= 1e-5 sqrt(A_ii A_jj), A = sum_k |w_k| y_k y_k^T) over operand scales in tests/test_gpu_cma_range.py.
 #include <cuda.h>
 #include <stddef.h>
 #include "des_common.cuh"
@@ -28,19 +34,63 @@ constexpr int kABytes = kBM * kBK * 2, kBBytes = kBN * kBK * 2;
 constexpr int kStageBytes = 2 * kABytes + 2 * kBBytes;             // A_hi | A_lo | B_hi | B_lo = 96 KB
 constexpr int kThreads = 6 * 32;
 
+// e_j is capped so that 2^e_j and 2^-e_j are normal floats and multiplying by them is exact; the cap only binds for
+// columns whose largest |z| is below 2^-112
+constexpr int kExpMax = 126;
+
+__device__ __forceinline__ float pow2f(int e) { return __int_as_float((127 + e) << 23); }     // 2^e for -126 <= e <= 127
+
+// ---- exponent pass: e_j such that max_k |sqrt|w_k| y_kj| * 2^e_j is in [2^14, 2^15) ------------------------------------
+// (hi is at most 2^15, so finite, and lo is a normal fp16 for entries within about 2^-17 of the column's largest).  A column
+// that is all zero, or holds an inf or NaN, gets e_j = 0: the non-finite value stays in row and column j.
+__global__ void __launch_bounds__(1024) cma_exponent_kernel(int *__restrict__ exps, const float *__restrict__ Y,
+                                                            const float *__restrict__ w, int64_t lambda, int64_t n) {
+    __shared__ float sqrt_w[1024];
+    __shared__ uint32_t part[32][33];
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;          // 32 columns x 32 slices of k
+    const int64_t j = (int64_t)blockIdx.x * 32 + tx;
+    // max of |z| as bit patterns: for non-negative floats their order is the order of the values, and NaN sorts above inf
+    uint32_t m = 0;
+    for (int64_t k0 = 0; k0 < lambda; k0 += 1024) {
+        // sqrt|w_k| from shared memory: with the sqrtf (and its slow-path call) out of the loop, the loads of Y batch up
+        __syncthreads();
+        sqrt_w[threadIdx.x] = k0 + threadIdx.x < lambda ? sqrtf(fabsf(__ldg(w + k0 + threadIdx.x))) : 0.f;
+        __syncthreads();
+        const int kn = (int)min((int64_t)1024, lambda - k0);
+        if (j < n) {
+            const float *y = Y + k0 * n + j;
+#pragma unroll 16
+            for (int r = ty; r < kn; r += 32) m = max(m, __float_as_uint(fabsf(sqrt_w[r] * __ldg(y + (int64_t)r * n))));
+        }
+    }
+    part[ty][tx] = m;
+    __syncthreads();
+    if (ty == 0 && j < n) {
+        for (int r = 1; r < 32; ++r) m = max(m, part[r][tx]);
+        int e = 0;
+        if (m != 0u && m < 0x7f800000u) {
+            const int lg = m >= 0x00800000u ? (int)(m >> 23) - 127 : -118 - __clz((int)m);   // floor(log2 max), subnormals too
+            e = min(14 - lg, kExpMax);
+        }
+        exps[j] = e;
+    }
+}
+
 // ---- pre-pass: transpose + scale + split --------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) cma_split_kernel(__half *__restrict__ zs_hi, __half *__restrict__ zs_lo,
                                                         __half *__restrict__ z_hi, __half *__restrict__ z_lo,
                                                         const float *__restrict__ Y, const float *__restrict__ w,
-                                                        int64_t lambda, int64_t lambda_pad, int64_t n) {
+                                                        const int *__restrict__ exps, int64_t lambda, int64_t lambda_pad,
+                                                        int64_t n) {
     __shared__ float tile[32][33];
     __shared__ float sgn[32];
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;          // 32 x 8
     const int64_t k0 = (int64_t)blockIdx.y * 32, j0 = (int64_t)blockIdx.x * 32;
+    const float scale = j0 + tx < n ? pow2f(__ldg(exps + j0 + tx)) : 1.f;
     for (int r = ty; r < 32; r += 8) {
         const int64_t k = k0 + r, j = j0 + tx;
         float v = 0.f;
-        if (k < lambda && j < n) v = sqrtf(fabsf(__ldg(w + k))) * __ldg(Y + k * n + j);
+        if (k < lambda && j < n) v = (sqrtf(fabsf(__ldg(w + k))) * __ldg(Y + k * n + j)) * scale;   // same z as the exponent pass
         tile[r][tx] = v;
     }
     if (threadIdx.x < 32) sgn[threadIdx.x] = (k0 + threadIdx.x < lambda && __ldg(w + k0 + threadIdx.x) < 0.f) ? -1.f : 1.f;
@@ -63,6 +113,7 @@ __global__ void __launch_bounds__(256) cma_split_kernel(__half *__restrict__ zs_
 
 struct Args {
     float *out;
+    const int *exps;         // e_j of the exponent pass
     int64_t n;
     int k_stages;            // lambda_pad / 64
     int tiles_m, tiles_n;    // 128-row and 256-column blocks
@@ -95,6 +146,7 @@ __device__ __forceinline__ bool elect_one() {
 struct Bars {
     uint64_t full[kStages], empty[kStages], acc_full;
     uint32_t tmem_base;
+    float unscale_col[kBN];  // 2^-e_j of the tile's columns
 };
 
 __global__ void __launch_bounds__(kThreads, 1) cma_syrk_kernel(Args a, const __grid_constant__ CUtensorMap map_a_hi,
@@ -176,11 +228,18 @@ __global__ void __launch_bounds__(kThreads, 1) cma_syrk_kernel(Args a, const __g
         }
     } else {
         // ---- epilogue: TMEM lane quadrant = warp id % 4; lane = output row
-        mbar_wait(smem_u32(&bars->acc_full), 0);
-        tc_fence_after();
         const int q = warp & 3;
         const int64_t i = (int64_t)bi * kBM + q * 32 + lane;
         const int64_t n = a.n;
+        // the unscaling factors of the tile's rows and columns are read while the MMAs run (padding beyond n: factor 1)
+        const float unscale_i = i < n ? pow2f(-__ldg(a.exps + i)) : 1.f;
+        for (int c = threadIdx.x - 64; c < kBN; c += kThreads - 64) {
+            const int64_t j = (int64_t)bj * kBN + c;
+            bars->unscale_col[c] = j < n ? pow2f(-__ldg(a.exps + j)) : 1.f;
+        }
+        asm volatile("bar.sync 1, %0;" ::"n"(kThreads - 64) : "memory");     // the four epilogue warps
+        mbar_wait(smem_u32(&bars->acc_full), 0);
+        tc_fence_after();
         const uint32_t taddr = tmem + ((uint32_t)(q * 32) << 16);
         // packed tiles are padded to a multiple of their side: the padding must be written too (zeros from the TMA fill)
         const int64_t jlimit = a.packed ? (int64_t)a.ptiles_per_side * a.ptile : n;
@@ -198,6 +257,11 @@ __global__ void __launch_bounds__(kThreads, 1) cma_syrk_kernel(Args a, const __g
 #pragma unroll
                 for (int e = 0; e < 32; ++e) v[e] = __float_as_uint(__uint_as_float(v[e]) + __uint_as_float(v2[e]));
             }
+            // undo S on both sides: two separate power-of-two multiplies, each exact (one factor 2^-(e_i + e_j) may not
+            // be a float)
+#pragma unroll
+            for (int e = 0; e < 32; ++e)
+                v[e] = __float_as_uint((__uint_as_float(v[e]) * unscale_i) * bars->unscale_col[c0 + e]);
             if (a.packed) {
                 // packed upper tiles of side ptile: element (i, j) lives in tile (i / ptile, j / ptile), bi' <= bj'
                 const int64_t pb_i = i / a.ptile, pb_j = j0 / a.ptile;
@@ -251,7 +315,8 @@ static int64_t lambda_pad_of(int64_t lambda) { return (lambda + kBK - 1) / kBK *
 
 extern "C" DES_API size_t des_cma_tc_workspace_bytes(int64_t n, int64_t lambda_local) {
     if (n <= 0 || lambda_local <= 0) return 0;
-    return 4 * (size_t)n * (size_t)des::cmatc::lambda_pad_of(lambda_local) * sizeof(__half) + 1024;
+    // Zs_hi | Zs_lo | Z_hi | Z_lo | e, after aligning the base to 1024 B
+    return 4 * (size_t)n * (size_t)des::cmatc::lambda_pad_of(lambda_local) * sizeof(__half) + (size_t)n * sizeof(int) + 1024;
 }
 
 extern "C" DES_API int des_cma_rank_mu_tc(float *out_dev, const float *Y_dev, const float *w_dev, int64_t lambda_local, int64_t n,
@@ -275,8 +340,11 @@ extern "C" DES_API int des_cma_rank_mu_tc(float *out_dev, const float *Y_dev, co
     const int64_t lp = lambda_pad_of(lambda_local);
     __half *base = reinterpret_cast<__half *>(((uintptr_t)workspace_dev + 1023) & ~(uintptr_t)1023);
     __half *zs_hi = base, *zs_lo = base + n * lp, *z_hi = base + 2 * n * lp, *z_lo = base + 3 * n * lp;
+    int *exps = reinterpret_cast<int *>(base + 4 * n * lp);
+    cma_exponent_kernel<<<(unsigned)((n + 31) / 32), 1024, 0, st>>>(exps, Y_dev, w_dev, lambda_local, n);
+    DES_LAUNCH_CHECK("cma_exponent_kernel");
     cma_split_kernel<<<dim3((unsigned)((n + 31) / 32), (unsigned)(lp / 32)), 256, 0, st>>>(zs_hi, zs_lo, z_hi, z_lo, Y_dev, w_dev,
-                                                                                          lambda_local, lp, n);
+                                                                                          exps, lambda_local, lp, n);
     DES_LAUNCH_CHECK("cma_split_kernel");
     CUtensorMap maps[4];
     __half *ptrs[4] = {zs_hi, zs_lo, z_hi, z_lo};
@@ -294,7 +362,7 @@ extern "C" DES_API int des_cma_rank_mu_tc(float *out_dev, const float *Y_dev, co
         }
     }
     Args a;
-    a.out = out_dev; a.n = n; a.k_stages = (int)(lp / kBK);
+    a.out = out_dev; a.exps = exps; a.n = n; a.k_stages = (int)(lp / kBK);
     a.tiles_m = (int)((n + kBM - 1) / kBM); a.tiles_n = (int)((n + kBN - 1) / kBN);
     a.packed = packed ? 1 : 0;
     a.ptile = n <= 2048 ? 64 : 128;

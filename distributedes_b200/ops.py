@@ -298,7 +298,8 @@ def _cma_rank_mu(Y, w, out, packed, path):
 
 def cma_rank_mu(Y, w, out=None, path=None):
     """dC[n,n] = sum_i w_i y_i y_i^T for Y[lambda_local, n] (rank-mu term of es.tell, cma_es.py:90).
-    path: None = tensor cores (split-fp16 tcgen05 SYRK) for n >= 256, fp32 FFMA below; 'tc' / 'ffma' force one."""
+    path: None = tensor cores (split-fp16 tcgen05 SYRK) for n >= CMA_TC_MIN_N (2048), fp32 FFMA below; 'tc' / 'ffma'
+    force one."""
     lam, n = Y.shape
     if w.numel() != lam:
         raise RuntimeError('w has %d entries, Y has %d rows' % (w.numel(), lam))

@@ -237,10 +237,13 @@ DES_API int des_cma_rank_mu_packed(float *tiles_out_dev, const float *Y_dev, con
 DES_API int des_cma_cov_apply_packed(float *C_dev, const float *tiles_dev, const float *pc_dev, int64_t n, double decay,
                                      double c1, double cmu, void *stream);
 
-/* The rank-mu term on the tensor cores (csrc/des_cma_tc.cu): dC = Zs^T Z with Z = diag(sqrt|w|) Y, operands split into
- * fp16 hi + lo (three tcgen05 MMAs per k-step, fp32 accumulation, TMA-fed) — same result contract as des_cma_rank_mu
- * (packed == 0: full symmetric [n][n]) / des_cma_rank_mu_packed (packed != 0), within 1e-5 of the fp64 restatement in both
- * norms.  Needs des_cma_tc_workspace_bytes(n, lambda_local) bytes of workspace; |sqrt|w_k| * y| must stay below 65504. */
+/* The rank-mu term on the tensor cores (csrc/des_cma_tc.cu): dC = Zs^T Z with Z = diag(sqrt|w|) Y, each coordinate j of Z
+ * scaled by a power of two 2^e_j (undone exactly on the output) so that its largest |entry| lies in [2^14, 2^15), then
+ * split into fp16 hi + lo (three tcgen05 MMAs per k-step, fp32 accumulation, TMA-fed) — same result contract as
+ * des_cma_rank_mu (packed == 0: full symmetric [n][n]) / des_cma_rank_mu_packed (packed != 0), within 1e-5 of the fp64
+ * restatement in both norms and entry by entry within 1e-5 sqrt(A_ii A_jj), A = sum_k |w_k| y_k y_k^T, at any scale of
+ * the coordinates.  An inf or NaN in coordinate j of Y reaches only row and column j.  Needs
+ * des_cma_tc_workspace_bytes(n, lambda_local) bytes of workspace. */
 DES_API size_t des_cma_tc_workspace_bytes(int64_t n, int64_t lambda_local);
 DES_API int des_cma_rank_mu_tc(float *out_dev, const float *Y_dev, const float *w_dev, int64_t lambda_local, int64_t n,
                                int packed, void *workspace_dev, size_t workspace_bytes, void *stream);
